@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- pose projections/s (forward + analytic d(dist)/d(pose) + step) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -22,6 +22,11 @@ the in-process FFMA2 micro-benchmark next to it; `roofline_hbm` is the north-sta
 C4 motion-denoise loop, C5 data-parallel train step).  `cpu_baseline` / `--impl reference` time the REFERENCE's own
 PoseNDF (oracle/_ref, an unmodified copy made by oracle/make_ref.py) on the host cores -- the only places that
 touch oracle/.
+
+`--dump-outputs DIR` (rank 0) writes what the last timed step returned to its caller: the gathered projected poses
+(DIR/projected_poses.npy, float32 [world*B, 21, 4]) and their distances (DIR/dist.npy, float32 [world*B, 1]).  Weights
+and poses are seeded, so two builds run with the same arguments can be compared output for output.  Above
+DUMP_BUDGET_BYTES the same fixed, seeded subset of poses is kept in both files (sorted pose order).
 """
 from __future__ import annotations
 
@@ -44,6 +49,7 @@ BATCH_PER_GPU = 65536
 FLOPS_PER_PROJECTION = 5_450_416      # SURVEY 8(d): 2*MAC, forward + input gradient
 BYTES_PER_PROJECTION = 676            # 336 in + 336 out + 4 dist
 WEIGHT_SEED, POSE_SEED = 1, 1234
+DUMP_BUDGET_BYTES, DUMP_SAMPLE_SEED = 60 << 20, 0      # array bytes: the .npy files, headers included, stay under 64 MB
 METRIC = "pose projections/s (fwd+grad+step)"
 UNIT = "poses/s"
 WORKLOAD = "configs[1]: 65 536-pose forward + d(dist)/d(pose) projection step per GPU, amass.yaml lrelu"
@@ -274,6 +280,17 @@ def run_other_configs(eng, dev, rank, world, gather):
     return out
 
 
+def dump_outputs(out_dir, arrays):
+    """write {name: array, poses on axis 0} as out_dir/<name>.npy; above DUMP_BUDGET_BYTES every array keeps the same fixed,
+    seeded subset of poses"""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    keep = DUMP_BUDGET_BYTES // sum(a.nbytes // n for a in arrays.values())
+    rows = np.sort(np.random.default_rng(DUMP_SAMPLE_SEED).choice(n, keep, replace=False)) if n > keep else slice(None)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a[rows])
+
+
 # ------------------------------------------------------------------------------------------------ main arm
 def main():
     ap = argparse.ArgumentParser()
@@ -285,7 +302,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the C3/C4/C5 legs")
     ap.add_argument("--gather", default="auto", choices=["auto", "peer", "nccl"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's projected poses and distances as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -348,6 +370,8 @@ def main():
     launches = eng.launch_count() - launches0
     ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = _max_over_ranks(sum(ms), dev, world)
+    if args.dump_outputs and rank == 0:      # before the e2e loop, which reuses x when N > 1
+        dump_outputs(args.dump_outputs, {"projected_poses": G.poses.cpu().numpy(), "dist": G.dist.cpu().numpy()})
 
     # ---- kernel-only time (no gather) for the roofline, same flush discipline: the path the library picks for this batch
     # (tensor-core DFNet, "tile 128") and the fused fp32-FMA kernel (tile 32) next to it
