@@ -277,12 +277,13 @@ int pndf_knn_exact(int device, const float* query_dev, int64_t Q, const float* d
  *     reference's real call sites, B = 10 in experiments/sample_poses.py:96);
  *   larger batches, quaternion input or the axis-angle prior mode (pndf_prior_grad, pndf_denoise_prior): the tensor-core engine
  *     ("tile 128": DFNet GEMMs as 3xTF32 tcgen05 kernels on 128-pose tiles, pndf_tc.cu);
- *   training exports, tangent launches, prior-mode batches above 131 072 poses: the fused FFMA kernel with 32-pose tiles (8-pose
- *     tiles while one round of them covers the batch).
+ *   training exports, tangent launches, the debug dump, prior-mode batches above 131 072 poses: the fused FFMA kernel with 32-pose
+ *     tiles.
  * The engines differ in fp32 summation order / split arithmetic (same parity bars), so a caller that splits ONE batch over several
  * launches or GPUs and wants bits identical to the unsplit run pins the tile the whole batch would get:
  * tile = pndf_tile_for_batch(h, B_total), pndf_set_tile_policy(h, tile), launches, pndf_set_tile_policy(h, 0).
- * posendf_b200/dist.py and pndf_project_host do this.  PNDF_TILE=8|32|128 in the environment overrides everything (tests, tuning). */
+ * posendf_b200/dist.py does this; pndf_project_host runs all its chunks at the tile of its whole batch by itself.
+ * PNDF_TILE=8|32|128 in the environment overrides everything (tests, tuning). */
 int pndf_set_tile_policy(pndf_handle* h, int tile);
 int pndf_tile_for_batch(pndf_handle* h, int64_t B, int* tile);
 

@@ -45,17 +45,12 @@ int fail(const std::string& msg) {
 const int kAmassDims[6] = {256, 512, 1024, 512, 256, 64};
 const double kSmallTileCost = 0.40;      // time of an 8-pose tile relative to a 32-pose tile (measured, DESIGN.md)
 const long long kTcChunk = 131072;       // poses per pass of the tensor-core path (5.7 GB of activations)
-// From one pose more than a single round of 8-pose tiles covers (8 x SMs = 1 184) the DFNet GEMMs run on the tensor cores
-// (pndf_tc.cu).  Measured, forward + d(dist)/d(pose) + step, lrelu (tools/small_batch_bench.py): 1 024 poses 195 us (8-pose tiles) vs
-// 252 us; 1 536: 389 vs 270 us; 4 736: 459 (32-pose tiles) vs 301 us; 8 192: 917 vs 412 us.
-inline bool tc_batch(const pndf_handle* h, long long B);
 
 }  // namespace
 
 struct pndf_handle {
     pndf_config cfg;
     int num_sms = 0;
-    bool no_tc = false;           // set while a caller runs launch chains side by side (the tensor-core engine has ONE set of buffers)
     bool have_weights = false;
     float* d_wstream = nullptr;   // slab stream
     size_t wstream_floats = 0;
@@ -108,10 +103,6 @@ struct pndf_handle {
     int tile_policy = 0;                 // 0: per launch from its batch size, 8 / 32 / 128: pinned (pndf_set_tile_policy); 128 = tensor-core path
     TcState* tc = nullptr;               // tensor-core DFNet path (pndf_tc.cu); nullptr if it could not be set up
 };
-
-namespace {
-inline bool tc_batch(const pndf_handle* h, long long B) { return B > 8LL * h->num_sms; }
-}  // namespace
 
 namespace {
 
@@ -234,11 +225,13 @@ __global__ void pack_gather_kernel(const float* __restrict__ flat, const int32_t
     }
 }
 
-int pack_on_device(pndf_handle* h, const float* d_flat, cudaStream_t st) {
-    // launches still reading the old weights on another stream must finish first
+// Rewrite the weights on `st`: `write()` enqueues the kernels that change the packed buffers, then the tensor-core copies are split
+// from the flat vector d_flat.  Launches still reading the old weights on another stream finish first; launches on another stream
+// wait for w_event (order_after_weights).
+template <class Write>
+int write_weights(pndf_handle* h, const float* d_flat, cudaStream_t st, Write write) {
     if (h->used && h->use_stream != st) CUDA_OK(cudaStreamWaitEvent(st, h->use_event, 0));
-    pack_gather_kernel<<<h->num_sms * 4, 256, 0, st>>>(d_flat, h->d_map_w, h->d_wstream, h->wstream_floats);
-    pack_gather_kernel<<<8, 256, 0, st>>>(d_flat, h->d_map_s, h->d_small, h->small_floats);
+    write();
     CUDA_OK(cudaGetLastError());
     if (h->tc && tc_set_weights(h->tc, d_flat, st)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
     if (!h->w_event) CUDA_OK(cudaEventCreateWithFlags(&h->w_event, cudaEventDisableTiming));
@@ -249,9 +242,26 @@ int pack_on_device(pndf_handle* h, const float* d_flat, cudaStream_t st) {
     return 0;
 }
 
+int pack_on_device(pndf_handle* h, const float* d_flat, cudaStream_t st) {
+    return write_weights(h, d_flat, st, [&] {
+        pack_gather_kernel<<<h->num_sms * 4, 256, 0, st>>>(d_flat, h->d_map_w, h->d_wstream, h->wstream_floats);
+        pack_gather_kernel<<<8, 256, 0, st>>>(d_flat, h->d_map_s, h->d_small, h->small_floats);
+    });
+}
+
 // a launch on a stream other than the one the weights were last repacked on has to wait for that repack
 int order_after_weights(pndf_handle* h, cudaStream_t st) {
     if (h->w_pending && st != h->w_stream) CUDA_OK(cudaStreamWaitEvent(st, h->w_event, 0));
+    return 0;
+}
+
+// Record that a launch on `st` reads the weights: a repack on another stream waits for it.  Not inside a stream capture (events
+// must not be recorded into one): the caller records after the graph launch.
+int mark_used(pndf_handle* h, cudaStream_t st) {
+    if (h->in_capture) return 0;
+    CUDA_OK(cudaEventRecord(h->use_event, st));
+    h->use_stream = st;
+    h->used = true;
     return 0;
 }
 
@@ -324,42 +334,44 @@ FusedFn fused_fn(int mode, bool dsoft, bool esoft, bool small_tile = false) {
     return esoft ? pndf_fused_entry_01(mode, small_tile) : pndf_fused_entry_00(mode, small_tile);
 }
 
-// Tile size of a launch.  A 32-pose tile per SM is the latency floor of the main kernel (~0.46 ms forward + reverse), so a batch
-// that cannot give every SM a tile runs the small-tile variant: 8 poses per tile, four times as many CTAs, each ~0.3-0.4 of
-// the time (the four lane groups split K).  It streams the weights once per 8 poses, so it only pays while the 32-pose tiling
-// needs a single round; `PNDF_TILE=8|32` in the environment forces a choice (tests, tuning).
+// Tile size of a launch: 8 or 32 poses per tile on the fused FFMA kernel, 128 = the tensor-core engine.  The engines and tilings
+// differ in fp32 summation order, so every bit-for-bit guarantee (sharded == unsharded, pndf_project_host == pndf_project, graph
+// replay == plain launches) rests on this one choice.
+//
+// The batch-size rule (pndf_tile_for_batch).  A 32-pose tile per SM is the latency floor of the fused kernel (~0.46 ms forward +
+// reverse), so a batch that cannot give every SM a tile runs the small-tile variant: 8 poses per tile, four times as many CTAs,
+// each ~0.3-0.4 of the time (the four lane groups split K).  It streams the weights once per 8 poses, so it only pays while the
+// 32-pose tiling needs a single round.  From one pose more than a single round of 8-pose tiles covers (8 x SMs = 1 184) the DFNet
+// GEMMs run on the tensor cores (pndf_tc.cu), ~3x the FFMA kernel (DESIGN.md 3b).  Measured, forward + d(dist)/d(pose) + step,
+// lrelu (tools/small_batch_bench.py): 1 024 poses 195 us (8-pose tiles) vs 252 us; 1 536: 389 vs 270 us; 4 736: 459 (32-pose
+// tiles) vs 301 us; 8 192: 917 vs 412 us.
 bool small_tile_for(const pndf_handle* h, long long B) {
     const long long t32 = (B + kTileM - 1) / kTileM, t8 = (B + 7) / 8;
     const long long r32 = (t32 + h->num_sms - 1) / h->num_sms, r8 = (t8 + h->num_sms - 1) / h->num_sms;
     return r32 == 1 && (double)r8 * kSmallTileCost < 0.9;
 }
-bool use_small_tile(const pndf_handle* h, const KParams& p, int mode) {
-    if (mode == 2 || p.dbg != nullptr || p.act_masks != nullptr) return false;
-    if (const char* e = getenv("PNDF_TILE")) return atoi(e) == 8;
-    if (h->tile_policy != 0) return h->tile_policy == 8;
-    return small_tile_for(h, p.B);
+int batch_tile(const pndf_handle* h, long long B) {
+    if (h->tc && B > 8LL * h->num_sms) return 128;
+    return small_tile_for(h, B) ? 8 : 32;
 }
-// Batches beyond one round of 8-pose tiles (forward, forward + gradient, projection steps on quaternions; the axis-angle prior and
-// the denoise loop) take the tensor-core engine: the DFNet GEMMs as 3xTF32 tcgen05 kernels, ~3x the FFMA kernel (DESIGN.md 3b).
-// Training exports, tangent launches, the debug dump and small batches stay on the fused FFMA kernel.
-// the engine a plain launch over B poses gets (environment override, pinned policy, batch size)
-bool tc_for_batch(const pndf_handle* h, long long B) {
-    if (!h->tc) return false;
-    if (const char* e = getenv("PNDF_TILE")) return atoi(e) == 128;
-    if (h->tile_policy != 0) return h->tile_policy == 128;
-    return tc_batch(h, B);
+// the tile a call over B poses asks for: `PNDF_TILE=8|32|128` in the environment (tests, tuning), else the pinned policy
+// (pndf_set_tile_policy), else the batch-size rule.  launch() narrows it to what the launch can take.
+int tile_for(const pndf_handle* h, long long B) {
+    if (const char* e = getenv("PNDF_TILE")) {
+        const int t = atoi(e);
+        return t == 8 ? 8 : (t == 128 && h->tc) ? 128 : 32;
+    }
+    if (h->tile_policy != 0) return h->tile_policy;
+    return batch_tile(h, B);
 }
-// axis-angle input = the prior mode (one evaluation + VJP, optionally with a denoise loop's pending Adam update in the prologue): on
-// the tensor-core engine as one pass (sequence bookkeeping does not survive the chunking of very large batches)
-bool tc_prior_ok(const KParams& p, int mode) {
+// Can the tensor-core engine take this launch?  Forward, forward + gradient and projection steps on quaternions, and the prior mode
+// (axis-angle input: one evaluation + VJP, optionally with a denoise loop's pending Adam update in the prologue) as ONE pass: the
+// sequence bookkeeping does not survive the chunking of very large batches.  Training exports, tangent launches and the debug dump
+// stay on the fused kernel.
+bool tc_capable(const pndf_handle* h, const KParams& p, int mode) {
+    if (!h->tc || mode == 2 || p.dbg != nullptr || p.act_masks != nullptr || p.tan_in != nullptr) return false;
+    if (p.input_kind == IN_QUAT && p.dn.pending == 0) return !(mode == 1 && p.steps > 1 && p.pose_out == nullptr);
     return mode == 1 && p.steps == 1 && !p.do_step && p.pose_out == nullptr && p.n_peers == 0 && p.B <= kTcChunk;
-}
-bool use_tc(const pndf_handle* h, const KParams& p, int mode) {
-    if (!h->tc || h->no_tc || mode == 2 || p.dbg != nullptr || p.act_masks != nullptr || p.tan_in != nullptr ||
-        (mode == 1 && p.steps > 1 && p.pose_out == nullptr))
-        return false;
-    if ((p.input_kind != IN_QUAT || p.dn.pending != 0) && !tc_prior_ok(p, mode)) return false;
-    return tc_for_batch(h, p.B);
 }
 
 int ensure_slot(pndf_handle* h, int slot) {
@@ -381,70 +393,50 @@ int ensure_encrows(pndf_handle* h, int64_t B) {
     return 0;
 }
 
-int launch(pndf_handle* h, KParams& p, int mode, cudaStream_t st, int slot = 0) {
+// One DFNet call at the tile its caller resolved (tile_for), narrowed to what the launch can take: 128 on a launch the tensor-core
+// engine cannot take runs the fused kernel with 32-pose tiles, and so does 8 on a tangent, export or debug launch.
+int launch(pndf_handle* h, KParams& p, int mode, int tile, cudaStream_t st, int slot = 0) {
     if (!h->have_weights) return fail("pndf_set_weights has not been called");
     if (p.B <= 0) return 0;
+    if ((tile == 128 && !tc_capable(h, p, mode)) || (tile == 8 && (mode == 2 || p.dbg != nullptr || p.act_masks != nullptr)))
+        tile = 32;
     p.wstream = h->d_wstream;
     for (int l = 0; l < 7; ++l) p.bias[l] = h->d_small + h->off_bias[l];
     p.w6 = h->d_small + h->off_w6;
     p.encw = h->cfg.use_enc ? h->d_small + h->off_enc : nullptr;
     p.dscratch = h->d_scratch[slot];
     p.z0scratch = h->d_z0[slot];
-    if (use_tc(h, p, mode)) {
-        TcArgs a;
-        a.pose_in = p.pose_in; a.pose_out = p.pose_out; a.dist = p.dist; a.grad = p.grad; a.g_up = p.g_up; a.B = p.B;
-        a.steps = p.steps; a.do_step = p.do_step; a.renorm = p.renorm; a.normalise = p.normalise; a.want_grad = (mode == 1);
-        a.encw = p.encw; a.w6 = p.w6; a.n_peers = p.n_peers;
-        for (int l = 0; l < 7; ++l) a.bias[l] = p.bias[l];
-        for (int r = 0; r < p.n_peers; ++r) { a.peer_pose[r] = p.peer_pose[r]; a.peer_dist[r] = p.peer_dist[r]; }
-        a.input_kind = p.input_kind;
-        a.dn = (p.dn.pending != 0) ? &p.dn : nullptr;
-        if (!h->in_capture && order_after_weights(h, st)) return 1;
-        if (p.input_kind != IN_QUAT) {      // prior mode: one pass (use_tc has checked B <= kTcChunk)
-            if (tc_run(h->tc, a, st, &h->launches)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
-            if (h->in_capture) return 0;
-            CUDA_OK(cudaEventRecord(h->use_event, st));
-            h->use_stream = st;
-            h->used = true;
-            return 0;
-        }
+    if (!h->in_capture && order_after_weights(h, st)) return 1;
+    if (tile == 128) {
         // the activations of the whole DFNet chain live in HBM between the layer kernels (43.5 KB per pose): bound them by walking
-        // very large batches in chunks of kTcChunk poses (every pose is independent; all steps of a chunk run before the next chunk)
+        // very large batches in chunks of kTcChunk poses (every pose is independent; all steps of a chunk run before the next chunk).
+        // The prior mode is one pass (tc_capable): its sequence bookkeeping (p.dn) is never sliced.
+        const long long row = (p.input_kind == IN_QUAT) ? 84 : 63;
         for (long long off = 0; off < p.B; off += kTcChunk) {
-            TcArgs c = a;
+            KParams c = p;
             c.B = std::min<long long>(kTcChunk, p.B - off);
-            c.pose_in = a.pose_in + off * 84;
-            if (a.pose_out) c.pose_out = a.pose_out + off * 84;
-            if (a.dist) c.dist = a.dist + off;
-            if (a.grad) c.grad = a.grad + off * 84;
-            if (a.g_up) c.g_up = a.g_up + off;
-            for (int r = 0; r < a.n_peers; ++r) {
-                c.peer_pose[r] = a.peer_pose[r] + off * 84;
-                if (a.peer_dist[r]) c.peer_dist[r] = a.peer_dist[r] + off;
+            c.pose_in = p.pose_in + off * row;
+            if (p.pose_out) c.pose_out = p.pose_out + off * row;
+            if (p.dist) c.dist = p.dist + off;
+            if (p.grad) c.grad = p.grad + off * row;
+            if (p.g_up) c.g_up = p.g_up + off;
+            for (int r = 0; r < p.n_peers; ++r) {
+                c.peer_pose[r] = p.peer_pose[r] + off * row;
+                if (p.peer_dist[r]) c.peer_dist[r] = p.peer_dist[r] + off;
             }
-            if (tc_run(h->tc, c, st, &h->launches)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
+            if (tc_run(h->tc, c, mode == 1, st, &h->launches)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
         }
-        if (h->in_capture) return 0;
-        CUDA_OK(cudaEventRecord(h->use_event, st));
-        h->use_stream = st;
-        h->used = true;
-        return 0;
+        return mark_used(h, st);
     }
-    const bool small = use_small_tile(h, p, mode);
-    p.ntiles = (int)(small ? (p.B + 7) / 8 : (p.B + kTileM - 1) / kTileM);
+    p.ntiles = (int)(tile == 8 ? (p.B + 7) / 8 : (p.B + kTileM - 1) / kTileM);
     p.use_enc = h->cfg.use_enc; p.enc_act = h->cfg.enc_act; p.df_act = h->cfg.df_act;
     p.enc_beta = h->cfg.enc_beta; p.df_beta = h->cfg.df_beta;
     p.f0_slabs = h->f0_slabs; p.z0_rows = h->z0_rows; p.in_dim = h->cfg.in_dim;
     const int grid = std::min(p.ntiles, h->num_sms);
-    if (!h->in_capture && order_after_weights(h, st)) return 1;
-    fused_fn(mode, h->cfg.df_act == PNDF_ACT_SOFTPLUS, h->cfg.enc_act == PNDF_ACT_SOFTPLUS, small)<<<grid, kThreads, kSmTotal, st>>>(p);
+    fused_fn(mode, h->cfg.df_act == PNDF_ACT_SOFTPLUS, h->cfg.enc_act == PNDF_ACT_SOFTPLUS, tile == 8)<<<grid, kThreads, kSmTotal, st>>>(p);
     CUDA_OK(cudaGetLastError());
     h->launches++;
-    if (h->in_capture) return 0;       // events must not be recorded into a capture; the caller records after the graph launch
-    CUDA_OK(cudaEventRecord(h->use_event, st));
-    h->use_stream = st;
-    h->used = true;
-    return 0;
+    return mark_used(h, st);
 }
 
 }  // namespace
@@ -548,7 +540,7 @@ int pndf_forward(pndf_handle* h, const float* pose_dev, int64_t B, int normalise
     CUDA_OK(cudaSetDevice(h->cfg.device));
     KParams p{};
     p.pose_in = pose_dev; p.dist = dist_dev; p.B = B; p.steps = 1; p.normalise = normalise; p.input_kind = IN_QUAT;
-    return launch(h, p, 0, (cudaStream_t)stream);
+    return launch(h, p, 0, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_forward_grad(pndf_handle* h, const float* pose_dev, int64_t B, int normalise, const float* g_up_dev,
@@ -560,7 +552,7 @@ int pndf_forward_grad(pndf_handle* h, const float* pose_dev, int64_t B, int norm
     KParams p{};
     p.pose_in = pose_dev; p.dist = dist_dev; p.grad = grad_dev; p.g_up = g_up_dev; p.B = B; p.steps = 1;
     p.normalise = normalise; p.input_kind = IN_QUAT;
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_project(pndf_handle* h, float* pose_dev, int64_t B, int steps, int renorm, float* dist_dev, void* stream) {
@@ -572,7 +564,7 @@ int pndf_project(pndf_handle* h, float* pose_dev, int64_t B, int steps, int reno
     KParams p{};
     p.pose_in = pose_dev; p.pose_out = pose_dev; p.dist = dist_dev; p.B = B; p.steps = steps; p.do_step = 1;
     p.renorm = renorm; p.normalise = 1; p.input_kind = IN_QUAT;
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_project_gather(pndf_handle* h, float* pose_dev, int64_t B, int steps, int renorm, float* dist_dev,
@@ -593,7 +585,7 @@ int pndf_project_gather(pndf_handle* h, float* pose_dev, int64_t B, int steps, i
         p.peer_pose[r] = peer_pose_dev[r];
         p.peer_dist[r] = peer_dist_dev ? peer_dist_dev[r] : nullptr;
     }
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 // ---- peer memory (one process per GPU): cudaMalloc + cudaIpc handles; the handle bytes travel through the caller's
@@ -657,7 +649,7 @@ int pndf_prior_grad(pndf_handle* h, const float* aa_dev, int64_t B, const float*
     KParams p{};
     p.pose_in = aa_dev; p.dist = dist_dev; p.grad = grad_aa_dev; p.g_up = g_up_dev; p.B = B; p.steps = 1;
     p.normalise = 1; p.input_kind = IN_AXIS_ANGLE;
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_project_host(pndf_handle* h, const float* pose_in_host, float* pose_out_host, float* dist_host, int64_t B,
@@ -667,21 +659,17 @@ int pndf_project_host(pndf_handle* h, const float* pose_in_host, float* pose_out
     if (B == 0) return 0;
     if (B < 0 || !pose_in_host || !pose_out_host) return fail("null argument");
     CUDA_OK(cudaSetDevice(h->cfg.device));
-    if (!h->hs[0]) {
-        for (int i = 0; i < 2; ++i) CUDA_OK(cudaStreamCreateWithFlags(&h->hs[i], cudaStreamNonBlocking));
-        if (cudaEventCreateWithFlags(&h->hs_ev, cudaEventDisableTiming) != cudaSuccess) h->hs_ev = nullptr;
-    }
+    for (int i = 0; i < 2; ++i)
+        if (!h->hs[i]) CUDA_OK(cudaStreamCreateWithFlags(&h->hs[i], cudaStreamNonBlocking));
+    if (!h->hs_ev) CUDA_OK(cudaEventCreateWithFlags(&h->hs_ev, cudaEventDisableTiming));
     if (ensure_slot(h, 1) || ensure_slot(h, 2)) return 1;   // the two streams overlap: each needs its own per-CTA scratch
-    // one tile size for all chunks, the one the whole batch would get: the result equals pndf_project on the same batch bit for bit
-    const int saved_policy = h->tile_policy;
-    if (saved_policy == 0) h->tile_policy = (h->tc && tc_batch(h, B)) ? 128 : (small_tile_for(h, B) ? 8 : 32);
-    struct Restore { pndf_handle* h; int v; ~Restore() { h->tile_policy = v; } } restore{h, saved_policy};
+    // one tile size for all chunks, the one the whole batch gets: the result equals pndf_project on the same batch bit for bit
+    const int tile = tile_for(h, B);
     // Chunk schedule.  Fused engine: uniform chunks of 4 tiles per SM (its time is linear in the tiles).  Tensor-core engine: its 15
     // launches per chunk want LARGE chunks (8 192 poses 0.41 ms, 49 152 poses 1.65 ms), but only the first chunk's upload and the
     // last chunk's download cannot hide under compute -- so a small head, large body chunks, a small tail.
     std::vector<int64_t> sizes;
-    const bool tc_chunks = (h->tile_policy == 128) && h->tc != nullptr && h->hs_ev != nullptr;
-    if (tc_chunks) {
+    if (tile == 128) {
         const int64_t kEdge = 8192, kBody = 49152;
         if (B <= 2 * kEdge) {
             for (int64_t off = 0; off < B; off += kEdge) sizes.push_back(std::min(kEdge, B - off));
@@ -719,10 +707,9 @@ int pndf_project_host(pndf_handle* h, const float* pose_in_host, float* pose_out
         p.steps = steps; p.do_step = 1; p.renorm = renorm; p.normalise = 1; p.input_kind = IN_QUAT;
         // the tensor-core path keeps its activations in ONE set of buffers per handle: its launches of consecutive chunks must not
         // overlap (the copies of the two streams still do)
-        const bool serial = (h->tile_policy == 128) && h->hs_ev != nullptr;
-        if (serial && off > 0) CUDA_OK(cudaStreamWaitEvent(st, h->hs_ev, 0));
-        if (launch(h, p, 1, st, 1 + which)) return 1;
-        if (serial) CUDA_OK(cudaEventRecord(h->hs_ev, st));
+        if (tile == 128 && off > 0) CUDA_OK(cudaStreamWaitEvent(st, h->hs_ev, 0));
+        if (launch(h, p, 1, tile, st, 1 + which)) return 1;
+        if (tile == 128) CUDA_OK(cudaEventRecord(h->hs_ev, st));
         CUDA_OK(cudaMemcpyAsync(pose_out_host + off * 84, h->d_chunk[which], nb * 84 * sizeof(float), cudaMemcpyDeviceToHost, st));
         if (dist_host) CUDA_OK(cudaMemcpyAsync(dist_host + off, h->d_chunk_dist[which], nb * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
@@ -784,11 +771,9 @@ int pndf_denoise_prior(pndf_handle* h, float* aa_dev, int64_t S, int64_t T, int 
     // SMs (config C4) leave the ninth round 90 % empty in every one of the 100 steps.
     // On the tensor-core engine (one set of activation buffers per handle) the loop is ONE chain over all sequences; its buffers
     // are reserved before the capture starts.
-    const bool on_tc = tc_for_batch(h, B) && B <= kTcChunk;
+    const bool on_tc = tile_for(h, B) == 128 && B <= kTcChunk;
     if (on_tc && tc_reserve(h->tc, B)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
     const int G = (!on_tc && S >= 2 && h->dn_stream2 != nullptr) ? 2 : 1;
-    struct NoTc { pndf_handle* h; bool v; ~NoTc() { h->no_tc = v; } } no_tc_guard{h, h->no_tc};
-    h->no_tc = !on_tc;            // two sequence groups = two concurrent chains: fused engine only
     auto enqueue = [&](cudaStream_t s0) -> int {
         if (cudaMemsetAsync(m, 0, (size_t)B * 63 * sizeof(float), s0) != cudaSuccess) return fail("cudaMemsetAsync failed");
         if (cudaMemsetAsync(v, 0, (size_t)B * 63 * sizeof(float), s0) != cudaSuccess) return fail("cudaMemsetAsync failed");
@@ -810,7 +795,9 @@ int pndf_denoise_prior(pndf_handle* h, float* aa_dev, int64_t S, int64_t T, int 
                     p.dn.ap = adam_of(t, (t - 1) / steps_per_iter);
                     p.dn.loss_out = loss_hist_dev ? loss_hist_dev + (size_t)(t - 1) * S + seq0[g] : nullptr;
                 }
-                if (launch(h, p, 1, sg[g], g)) return 1;
+                // off the tensor-core chain the groups run side by side: fused engine only
+                const int tile = tile_for(h, Bg);
+                if (launch(h, p, 1, (!on_tc && tile == 128) ? 32 : tile, sg[g], g)) return 1;
             }
         }
         for (int g = 0; g < G; ++g) {
@@ -855,10 +842,7 @@ int pndf_denoise_prior(pndf_handle* h, float* aa_dev, int64_t S, int64_t T, int 
         }
     }
     if (!graphed && enqueue(st)) return 1;
-    CUDA_OK(cudaEventRecord(h->use_event, st));
-    h->use_stream = st;
-    h->used = true;
-    return 0;
+    return mark_used(h, st);
 }
 
 int pndf_debug_dump_floats(size_t* n) {
@@ -873,7 +857,7 @@ int pndf_forward_grad_debug(pndf_handle* h, const float* pose_dev, int64_t B, in
     KParams p{};
     p.pose_in = pose_dev; p.dist = dist_dev; p.grad = grad_dev; p.B = std::min<int64_t>(B, 32); p.steps = 1;
     p.normalise = normalise; p.input_kind = IN_QUAT; p.dbg = dump_dev;
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_act_handoff_bytes(const pndf_handle* h, int64_t B, size_t* n) {
@@ -893,7 +877,7 @@ int pndf_forward_grad_export(pndf_handle* h, const float* pose_dev, int64_t B, i
     p.pose_in = pose_dev; p.dist = dist_dev; p.grad = grad_dev; p.B = B; p.steps = 1;
     p.normalise = normalise; p.input_kind = IN_QUAT; p.dbg = dump_dev; p.dump_all = 1;
     p.act_masks = (uint8_t*)act_handoff_dev;
-    return launch(h, p, 1, (cudaStream_t)stream);
+    return launch(h, p, 1, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_forward_tangent_export(pndf_handle* h, const float* pose_dev, int64_t B, int normalise, const float* tan_dev,
@@ -906,7 +890,7 @@ int pndf_forward_tangent_export(pndf_handle* h, const float* pose_dev, int64_t B
     p.pose_in = pose_dev; p.B = B; p.steps = 1; p.normalise = normalise; p.input_kind = IN_QUAT;
     p.dbg = dump_dev; p.dump_all = 1; p.tan_in = tan_dev;
     p.act_masks = (uint8_t*)act_handoff_dev;
-    return launch(h, p, 2, (cudaStream_t)stream);
+    return launch(h, p, 2, tile_for(h, p.B), (cudaStream_t)stream);
 }
 
 int pndf_encoder_tangent(pndf_handle* h, const float* pose_dev, const float* v_dev, int64_t B, int normalise,
@@ -1110,8 +1094,6 @@ int pndf_adam_step(pndf_handle* h, float* param_flat_dev, const float* grad_flat
     if (step < 1) return fail("pndf_adam_step: step counts from 1");
     CUDA_OK(cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
-    // launches of other streams still reading the packed weights must finish first (same rule as a repack)
-    if (h->used && h->use_stream != st) CUDA_OK(cudaStreamWaitEvent(st, h->use_event, 0));
     AdamStepParams p{};
     p.param = param_flat_dev; p.grad = grad_flat_dev; p.m = exp_avg_dev; p.v = exp_avg_sq_dev; p.n = (long long)n;
     p.lr_over_bias1 = (float)(lr / (1.0 - std::pow(beta1, (double)step)));
@@ -1119,14 +1101,7 @@ int pndf_adam_step(pndf_handle* h, float* param_flat_dev, const float* grad_flat
     p.one_minus_beta1 = (float)(1.0 - beta1); p.beta2 = (float)beta2; p.one_minus_beta2 = (float)(1.0 - beta2);
     p.eps = (float)eps; p.weight_decay = (float)weight_decay; p.grad_scale = (float)grad_scale;
     p.pos_a = h->d_pos[0]; p.pos_b = h->d_pos[1]; p.pos_s = h->d_pos[2]; p.wstream = h->d_wstream; p.small = h->d_small;
-    adam_step_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p);
-    CUDA_OK(cudaGetLastError());
-    if (h->tc && tc_set_weights(h->tc, param_flat_dev, st)) return fail(std::string("tensor-core path: ") + tc_last_error(h->tc));
-    if (!h->w_event) CUDA_OK(cudaEventCreateWithFlags(&h->w_event, cudaEventDisableTiming));
-    CUDA_OK(cudaEventRecord(h->w_event, st));
-    h->w_stream = st;
-    h->w_pending = true;
-    h->have_weights = true;
+    if (write_weights(h, param_flat_dev, st, [&] { adam_step_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p); })) return 1;
     h->launches++;
     return 0;
 }
@@ -1240,7 +1215,7 @@ int pndf_set_tile_policy(pndf_handle* h, int tile) {
 }
 int pndf_tile_for_batch(pndf_handle* h, int64_t B, int* tile) {
     if (!h || !tile || B < 0) return fail("bad argument");
-    *tile = (h->tc && tc_batch(h, B)) ? 128 : (small_tile_for(h, B) ? 8 : 32);
+    *tile = batch_tile(h, B);
     return 0;
 }
 

@@ -598,7 +598,7 @@ static int launch_gemm(TcState* s, const float* a_hi, const float* a_lo, long lo
     return tc_check(s, "tc_gemm_kernel launch");
 }
 
-int tc_run(TcState* s, const TcArgs& a, cudaStream_t st, int64_t* launches) {
+int tc_run(TcState* s, const KParams& a, int want_grad, cudaStream_t st, int64_t* launches) {
     if (a.input_kind != IN_QUAT && (a.steps != 1 || a.do_step || a.pose_out != nullptr))
         return tc_fail(s, "tensor-core path: axis-angle input is the prior mode (one evaluation, no step)");
     if (ensure_act(s, a.B)) return 1;
@@ -627,8 +627,8 @@ int tc_run(TcState* s, const TcArgs& a, cudaStream_t st, int64_t* launches) {
         ep.pose = pose_cur; ep.encw = a.encw; ep.z0_hi = zhi(0); ep.z0_lo = zlo(0); ep.B = a.B; ep.z0_ld = zw[0];
         ep.normalise = a.normalise; ep.use_enc = cfg.use_enc; ep.enc_act = cfg.enc_act; ep.enc_beta = cfg.enc_beta;
         ep.input_kind = a.input_kind;
-        if (a.dn != nullptr) ep.dn = *a.dn;
-        ep.feat_out = a.want_grad ? featp : nullptr;
+        if (a.dn.pending) ep.dn = a.dn;
+        ep.feat_out = want_grad ? featp : nullptr;
         if (esoft) tc_enc_kernel<true, false><<<tiles32, 256, enc_sm_total<false>(), st>>>(ep);
         else tc_enc_kernel<false, false><<<tiles32, 256, enc_sm_total<false>(), st>>>(ep);
         if (tc_check(s, "tc_enc_kernel (forward) launch")) return 1;
@@ -641,7 +641,7 @@ int tc_run(TcState* s, const TcArgs& a, cudaStream_t st, int64_t* launches) {
                 return (N % 128 == 0) ? launch_gemm<128>(s, zhi(l), zlo(l), P, s->kpad[l], bh, bl, N, fe, st)
                                       : launch_gemm<64>(s, zhi(l), zlo(l), P, s->kpad[l], bh, bl, N, fe, st);
             };
-            uint32_t* mk = (l < 5 && a.want_grad) ? maskp(l + 1) : nullptr;
+            uint32_t* mk = (l < 5 && want_grad) ? maskp(l + 1) : nullptr;
             const int rc = dsoft ? fwd(FwdEpi<true>{a.bias[l], zhi(l + 1), zlo(l + 1), zw[l + 1], dpar, nullptr})
                                  : fwd(FwdEpi<false>{a.bias[l], zhi(l + 1), zlo(l + 1), zw[l + 1], dpar, mk});
             if (rc) return 1;
@@ -650,11 +650,11 @@ int tc_run(TcState* s, const TcArgs& a, cudaStream_t st, int64_t* launches) {
         hp.z6_hi = zhi(6); hp.z6_lo = zlo(6); hp.w6 = a.w6; hp.b6 = a.bias[6]; hp.g_up = a.g_up; hp.B = a.B;
         hp.dist = last ? a.dist : nullptr; hp.dist_keep = dkeep; hp.soft = dsoft ? 1 : 0; hp.slope = dsoft ? 0.0f : dpar; hp.beta = cfg.df_beta;
         if (last) { hp.n_peers = a.n_peers; for (int r = 0; r < a.n_peers; ++r) hp.peer_dist[r] = a.peer_dist[r]; }
-        if (a.want_grad) { hp.t5_hi = thi(5); hp.t5_lo = tlo(5); }
+        if (want_grad) { hp.t5_hi = thi(5); hp.t5_lo = tlo(5); }
         tc_head_kernel<<<(unsigned)((a.B + 127) / 128), 128, 0, st>>>(hp);
         if (tc_check(s, "tc_head_kernel launch")) return 1;
         if (launches) *launches += 8;
-        if (!a.want_grad) break;
+        if (!want_grad) break;
         // ---- reverse chain: op l maps t_l (width n_out[l]) through W_l to the input side (width n_in[l])
         for (int l = 5; l >= 0; --l) {
             const float* bh = s->w_hi + s->r_off[l];

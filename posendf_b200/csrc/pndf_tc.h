@@ -10,32 +10,16 @@
 namespace pndf {
 
 struct TcState;
-struct DenoiseFuse;      // pndf_kernel.cuh
-
-struct TcArgs {
-    const float* pose_in = nullptr;   // [B][84] quaternion poses, or [B][63] axis-angle (input_kind = 1: prior mode, one evaluation, no step)
-    float* pose_out = nullptr;        // [B][84] (projection) or nullptr
-    float* dist = nullptr;            // [B] or nullptr
-    float* grad = nullptr;            // [B][84] ([B][63] in prior mode: the VJP to axis-angle) or nullptr
-    const float* g_up = nullptr;      // [B] or nullptr
-    long long B = 0;
-    int steps = 1, do_step = 0, renorm = 0, normalise = 1, want_grad = 1;
-    const float* encw = nullptr;      // encoder parameters (reference order) or nullptr
-    const float* bias[7] = {};        // dfnet.lin{l}.bias
-    const float* w6 = nullptr;        // dfnet.lin6.weight
-    float* peer_pose[7] = {};         // fused gather (see KParams)
-    float* peer_dist[7] = {};
-    int n_peers = 0;
-    int input_kind = 0;               // IN_QUAT / IN_AXIS_ANGLE (pndf_kernel.cuh)
-    const DenoiseFuse* dn = nullptr;  // denoise loop: the Adam update of the previous step, applied in the prologue of the first kernel
-};
+struct KParams;          // pndf_kernel.cuh
 
 int tc_create(TcState** out, const pndf_config* cfg);
 void tc_destroy(TcState* s);
 // split the flat fp32 parameter vector (reference order, device pointer) into the tf32 hi / lo weight copies; stream-ordered
 int tc_set_weights(TcState* s, const float* flat_dev, cudaStream_t st);
-// forward (want_grad = 0), forward + gradient, or `steps` projection steps; *launches is increased by the kernels launched
-int tc_run(TcState* s, const TcArgs& a, cudaStream_t st, int64_t* launches);
+// forward (want_grad = 0), forward + gradient, or a.steps projection steps over a.B poses, all in one pass; the weights come from
+// this state, the biases, lin6 and the encoder from a, and the previous denoise step's Adam update from a.dn when it is pending
+// (prior mode: axis-angle input, one evaluation, no step).  *launches is increased by the kernels launched
+int tc_run(TcState* s, const KParams& a, int want_grad, cudaStream_t st, int64_t* launches);
 // make sure the activation buffers hold B poses (allocates: call it BEFORE a stream capture that contains tc_run)
 int tc_reserve(TcState* s, long long B);
 const char* tc_last_error(TcState* s);

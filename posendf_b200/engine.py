@@ -138,13 +138,13 @@ class Engine:
         return dist, grad, dump
 
     def tile_for_batch(self, B) -> int:
-        """tile size (8 or 32 poses) the library would pick for a batch of B poses"""
+        """tile size the library's batch-size rule picks for B poses: 8 or 32 (fused FFMA kernel) or 128 (tensor-core engine)"""
         t = C.c_int()
         _lib.check(self.lib.pndf_tile_for_batch(self._h, int(B), C.byref(t)))
         return t.value
 
     def set_tile_policy(self, tile=0):
-        """0 = per launch from its batch size; 8 / 32 = pinned (split batches that must match the unsplit run bit for bit)"""
+        """0 = per launch from its batch size; 8 / 32 / 128 = pinned (split batches that must match the unsplit run bit for bit)"""
         _lib.check(self.lib.pndf_set_tile_policy(self._h, int(tile)))
 
     def launch_count(self) -> int:

@@ -17,7 +17,7 @@ CASES = golden_case_names()
 def tile_size(request, monkeypatch):
     """every test of this file runs with the library's own choice of path (tensor-core DFNet for large batches, 32-pose FFMA tiles,
     8-pose small-tile kernels for batches that cannot fill the SMs) and with each of them forced (PNDF_TILE = 128 / 32 / 8,
-    csrc/pndf_capi.cu::use_tc / use_small_tile)"""
+    csrc/pndf_capi.cu::tile_for)"""
     if request.param == "auto":
         monkeypatch.delenv("PNDF_TILE", raising=False)
     else:
