@@ -7,7 +7,8 @@
  * sizes, ints.  No torch types, no exceptions across the ABI.
  *
  * Conventions
- *   - return value: 0 = ok, non-zero = error (message via pndf_last_error(), thread-local).
+ *   - return value: 0 = ok, non-zero = error (message via pndf_last_error(), thread-local).  An error return, a failed
+ *     allocation included, leaves the handle usable.
  *   - "dev" pointers are CUDA device pointers on the handle's device, contiguous fp32, 16-byte aligned.
  *   - `stream` is a cudaStream_t passed as void* (NULL = default stream); all device work is enqueued
  *     on it, nothing synchronises implicitly, the caller owns every buffer it passes in.

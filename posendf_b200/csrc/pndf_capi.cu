@@ -8,6 +8,7 @@
 #include "pndf_wgrad.cuh"
 #include "pndf_feed.cuh"
 #include "pndf_tc.h"
+#include "pndf_host.h"
 #include "pndf_knn.cuh"
 
 #include <algorithm>
@@ -29,13 +30,16 @@ FusedFn pndf_fused_entry_11(int mode, int small_tile);
 }  // namespace pndf
 
 namespace {
-
 thread_local std::string g_err;
+}  // namespace
 
-int fail(const std::string& msg) {
+int pndf::fail(const std::string& msg) {
     g_err = msg;
     return 1;
 }
+
+namespace {
+
 #define CUDA_OK(expr)                                                                                     \
     do {                                                                                                  \
         cudaError_t _e = (expr);                                                                          \
@@ -52,14 +56,11 @@ struct pndf_handle {
     pndf_config cfg;
     int num_sms = 0;
     bool have_weights = false;
-    float* d_wstream = nullptr;   // slab stream
-    size_t wstream_floats = 0;
-    float* d_small = nullptr;     // biases (2625) + w6 (64) + encoder (3516), each 16B-aligned
-    size_t small_floats = 0;
+    DevBuf<float> d_wstream;      // slab stream
+    DevBuf<float> d_small;        // biases (2625) + w6 (64) + encoder (3516), each 16B-aligned
     // device-side packing: slab stream / small buffer element -> index into the flat parameter vector (-1 = zero pad)
-    int32_t* d_map_w = nullptr;
-    int32_t* d_map_s = nullptr;
-    float* d_flat = nullptr;      // staging copy of the flat parameter vector (host uploads)
+    DevBuf<int32_t> d_map_w, d_map_s;
+    DevBuf<float> d_flat;         // staging copy of the flat parameter vector (host uploads)
     cudaEvent_t w_event = nullptr; // recorded after the last repack; launches on other streams wait for it
     cudaStream_t w_stream = nullptr;
     bool w_pending = false;
@@ -69,8 +70,8 @@ struct pndf_handle {
     // floats), indexed by blockIdx only -- so every stream that may have a launch in flight needs its own copy:
     // slot 0 = the caller's stream (a handle is driven from ONE caller stream, include/pndf.h), slots 1, 2 = the two
     // pipeline streams of pndf_project_host (allocated on first use)
-    float* d_scratch[3] = {nullptr, nullptr, nullptr};
-    float* d_z0[3] = {nullptr, nullptr, nullptr};
+    DevBuf<float> d_scratch[3];
+    DevBuf<float> d_z0[3];
     cudaEvent_t use_event = nullptr;   // recorded after every launch: a repack on another stream waits for it (WAR on the weights)
     cudaStream_t use_stream = nullptr;
     bool used = false;
@@ -79,22 +80,17 @@ struct pndf_handle {
     // host pipeline (pndf_project_host)
     cudaStream_t hs[2] = {nullptr, nullptr};
     cudaEvent_t hs_ev = nullptr;
-    float* d_chunk[2] = {nullptr, nullptr};
-    float* d_chunk_dist[2] = {nullptr, nullptr};
-    int64_t chunk_poses = 0;
+    DevBuf<float> d_chunk[2];         // [chunk poses][84]
+    DevBuf<float> d_chunk_dist[2];
     // training (pndf_train_losses / pndf_wgrad_accumulate / pndf_adam_step)
-    int32_t* d_pos[3] = {nullptr, nullptr, nullptr};   // flat parameter index -> slab-stream position (forward / reverse copy), small-buffer position
-    float* d_ws = nullptr;            // split-K workspace [slots][n_params]
-    int ws_slots = 0;
-    float* d_encrows = nullptr;       // encoder-gradient rows [2][warps][kEncFloats]
-    long long encrow_warps = 0;
-    float* d_loss_partial = nullptr;  // [blocks][2]
-    int loss_blocks = 0;
-    unsigned int* d_loss_counter = nullptr;
-    double* d_loss_totals = nullptr;  // [3]
-    // denoise loop state (pndf_denoise_prior): raw gradient, Adam moments, dist
-    float* d_dn[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // + second distance buffer
-    int64_t dn_poses = 0;
+    DevBuf<int32_t> d_pos[3];         // flat parameter index -> slab-stream position (forward / reverse copy), small-buffer position
+    DevBuf<float> d_ws;               // split-K workspace [slots][n_params]
+    DevBuf<float> d_encrows;          // encoder-gradient rows [2][warps][kEncFloats] + first-level partial sums [2][kEncChunks][kEncFloats]
+    DevBuf<float> d_loss_partial;     // [blocks][2]
+    DevBuf<unsigned int> d_loss_counter;
+    DevBuf<double> d_loss_totals;     // [3]
+    // denoise loop state (pndf_denoise_prior): raw gradient, Adam moments ([poses][63] each), dist + second distance buffer
+    DevBuf<float> d_dn[5];
     cudaStream_t cap_stream = nullptr;   // graph capture of the denoise loop
     cudaStream_t dn_stream2 = nullptr;   // second sequence group of the denoise loop (parallel branch)
     cudaEvent_t dn_ev[2] = {nullptr, nullptr};
@@ -118,16 +114,7 @@ int validate(const pndf_config* c) {
     return 0;
 }
 
-size_t param_count(const pndf_config* c) {
-    size_t n = c->use_enc ? (size_t)kEncFloats : 0;
-    int prev = c->in_dim;
-    for (int l = 0; l < 6; ++l) {
-        n += (size_t)prev * c->dims[l] + c->dims[l];
-        prev = c->dims[l];
-    }
-    n += prev + 1;
-    return n;
-}
+size_t param_count(const pndf_config* c) { return (size_t)ParamLayout(*c).total; }
 
 // Append one op's weights in the per-warp slab order the kernel consumes (pndf_kernel.cuh): for each slab index,
 // for each of the 8 warps, R rows x FW feature columns (R*FW = 1024).  TN = features per thread, KG = K-groups.
@@ -159,19 +146,13 @@ void pack_op(std::vector<float>& out, int K, int TN, int KG, F get) {
 // actual packing of weights is then a device-side gather (pack_gather_kernel), which keeps a training step free of
 // host round trips.
 int build_streams(pndf_handle* h, const float* flat, std::vector<float>& s, std::vector<float>& sm) {
-    const float* enc = nullptr;
-    const float* cur = flat;
-    if (h->cfg.use_enc) {
-        enc = cur;
-        cur += kEncFloats;
-    }
-    const int in0 = h->cfg.in_dim;
-    const int widths[8] = {in0, 256, 512, 1024, 512, 256, 64, 1};
+    const ParamLayout L(h->cfg);
+    const int* widths = L.width;
     const float* W[7];
     const float* Bv[7];
     for (int l = 0; l < 7; ++l) {
-        W[l] = cur; cur += (size_t)widths[l + 1] * widths[l];
-        Bv[l] = cur; cur += widths[l + 1];
+        W[l] = flat + L.w_off[l];
+        Bv[l] = flat + L.b_off[l];
     }
     // ---- slab stream, in consumption order (pndf_kernel.cuh)
     s.clear();
@@ -213,7 +194,7 @@ int build_streams(pndf_handle* h, const float* flat, std::vector<float>& s, std:
     }
     align4(); h->off_w6 = sm.size(); sm.insert(sm.end(), W[6], W[6] + 64);
     align4(); h->off_enc = sm.size();
-    if (enc) sm.insert(sm.end(), enc, enc + kEncFloats);
+    sm.insert(sm.end(), flat, flat + L.enc_floats);
     align4();
     return 0;
 }
@@ -244,8 +225,8 @@ int write_weights(pndf_handle* h, const float* d_flat, cudaStream_t st, Write wr
 
 int pack_on_device(pndf_handle* h, const float* d_flat, cudaStream_t st) {
     return write_weights(h, d_flat, st, [&] {
-        pack_gather_kernel<<<h->num_sms * 4, 256, 0, st>>>(d_flat, h->d_map_w, h->d_wstream, h->wstream_floats);
-        pack_gather_kernel<<<8, 256, 0, st>>>(d_flat, h->d_map_s, h->d_small, h->small_floats);
+        pack_gather_kernel<<<h->num_sms * 4, 256, 0, st>>>(d_flat, h->d_map_w.get(), h->d_wstream.get(), h->d_wstream.size());
+        pack_gather_kernel<<<8, 256, 0, st>>>(d_flat, h->d_map_s.get(), h->d_small.get(), h->d_small.size());
     });
 }
 
@@ -273,15 +254,12 @@ int build_maps(pndf_handle* h) {
     std::vector<int32_t> mw(s.size()), ms(sm.size());
     for (size_t i = 0; i < s.size(); ++i) mw[i] = (int32_t)s[i] - 1;
     for (size_t i = 0; i < sm.size(); ++i) ms[i] = (int32_t)sm[i] - 1;
-    h->wstream_floats = s.size();
-    h->small_floats = sm.size();
-    CUDA_OK(cudaMalloc(&h->d_wstream, s.size() * sizeof(float)));
-    CUDA_OK(cudaMalloc(&h->d_small, sm.size() * sizeof(float)));
-    CUDA_OK(cudaMalloc(&h->d_map_w, mw.size() * sizeof(int32_t)));
-    CUDA_OK(cudaMalloc(&h->d_map_s, ms.size() * sizeof(int32_t)));
-    CUDA_OK(cudaMalloc(&h->d_flat, n * sizeof(float)));
-    CUDA_OK(cudaMemcpy(h->d_map_w, mw.data(), mw.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    CUDA_OK(cudaMemcpy(h->d_map_s, ms.data(), ms.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    if (h->d_wstream.reserve(s.size(), "slab stream") || h->d_small.reserve(sm.size(), "small-parameter buffer") ||
+        h->d_map_w.reserve(mw.size(), "slab-stream map") || h->d_map_s.reserve(ms.size(), "small-parameter map") ||
+        h->d_flat.reserve(n, "flat parameter staging buffer"))
+        return 1;
+    CUDA_OK(cudaMemcpy(h->d_map_w.get(), mw.data(), mw.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    CUDA_OK(cudaMemcpy(h->d_map_s.get(), ms.data(), ms.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     // inverse maps for the optimizer kernel: where does flat parameter i live in the packed buffers?
     std::vector<int32_t> pos[3];
     for (auto& v : pos) v.assign(n, -1);
@@ -296,8 +274,8 @@ int build_maps(pndf_handle* h) {
     for (size_t i = 0; i < n; ++i)
         if (pos[0][i] < 0 && pos[2][i] < 0) return fail("internal: a parameter is missing from the packed buffers");
     for (int k = 0; k < 3; ++k) {
-        CUDA_OK(cudaMalloc(&h->d_pos[k], n * sizeof(int32_t)));
-        CUDA_OK(cudaMemcpy(h->d_pos[k], pos[k].data(), n * sizeof(int32_t), cudaMemcpyHostToDevice));
+        if (h->d_pos[k].reserve(n, "optimizer position map")) return 1;
+        CUDA_OK(cudaMemcpy(h->d_pos[k].get(), pos[k].data(), n * sizeof(int32_t), cudaMemcpyHostToDevice));
     }
     return 0;
 }
@@ -375,22 +353,15 @@ bool tc_capable(const pndf_handle* h, const KParams& p, int mode) {
 }
 
 int ensure_slot(pndf_handle* h, int slot) {
-    if (!h->d_z0[slot]) CUDA_OK(cudaMalloc(&h->d_z0[slot], (size_t)h->num_sms * 128 * 32 * sizeof(float)));
-    if (h->cfg.df_act == PNDF_ACT_SOFTPLUS && !h->d_scratch[slot])
-        CUDA_OK(cudaMalloc(&h->d_scratch[slot], (size_t)h->num_sms * kUnits * 32 * sizeof(float)));
+    if (h->d_z0[slot].reserve((size_t)h->num_sms * 128 * 32, "per-CTA encoder scratch")) return 1;
+    if (h->cfg.df_act == PNDF_ACT_SOFTPLUS && h->d_scratch[slot].reserve((size_t)h->num_sms * kUnits * 32, "per-CTA softplus scratch"))
+        return 1;
     return 0;
 }
 
-int ensure_encrows(pndf_handle* h, int64_t B) {
-    const long long nwarps = ((B + 127) / 128) * 4;
-    if (h->encrow_warps < nwarps) {
-        cudaFree(h->d_encrows);
-        h->d_encrows = nullptr;
-        // per-warp rows [2][nwarps][E] followed by the first-level partial sums [2][kEncChunks][E]
-        CUDA_OK(cudaMalloc(&h->d_encrows, ((size_t)2 * nwarps + 2 * kEncChunks) * kEncFloats * sizeof(float)));
-        h->encrow_warps = nwarps;
-    }
-    return 0;
+// per-warp rows [2][nwarps][E] followed by the first-level partial sums [2][kEncChunks][E]
+int ensure_encrows(pndf_handle* h, long long nwarps) {
+    return h->d_encrows.reserve(((size_t)2 * nwarps + 2 * kEncChunks) * kEncFloats, "encoder-gradient rows");
 }
 
 // One DFNet call at the tile its caller resolved (tile_for), narrowed to what the launch can take: 128 on a launch the tensor-core
@@ -400,12 +371,12 @@ int launch(pndf_handle* h, KParams& p, int mode, int tile, cudaStream_t st, int 
     if (p.B <= 0) return 0;
     if ((tile == 128 && !tc_capable(h, p, mode)) || (tile == 8 && (mode == 2 || p.dbg != nullptr || p.act_masks != nullptr)))
         tile = 32;
-    p.wstream = h->d_wstream;
-    for (int l = 0; l < 7; ++l) p.bias[l] = h->d_small + h->off_bias[l];
-    p.w6 = h->d_small + h->off_w6;
-    p.encw = h->cfg.use_enc ? h->d_small + h->off_enc : nullptr;
-    p.dscratch = h->d_scratch[slot];
-    p.z0scratch = h->d_z0[slot];
+    p.wstream = h->d_wstream.get();
+    for (int l = 0; l < 7; ++l) p.bias[l] = h->d_small.get() + h->off_bias[l];
+    p.w6 = h->d_small.get() + h->off_w6;
+    p.encw = h->cfg.use_enc ? h->d_small.get() + h->off_enc : nullptr;
+    p.dscratch = h->d_scratch[slot].get();
+    p.z0scratch = h->d_z0[slot].get();
     if (!h->in_capture && order_after_weights(h, st)) return 1;
     if (tile == 128) {
         // the activations of the whole DFNet chain live in HBM between the layer kernels (43.5 KB per pose): bound them by walking
@@ -482,37 +453,18 @@ int pndf_create(const pndf_config* cfg, pndf_handle** out) {
 int pndf_destroy(pndf_handle* h) {
     if (!h) return 0;
     cudaSetDevice(h->cfg.device);
-    cudaFree(h->d_wstream);
-    cudaFree(h->d_small);
-    cudaFree(h->d_map_w);
-    cudaFree(h->d_map_s);
-    cudaFree(h->d_flat);
     if (h->w_event) cudaEventDestroy(h->w_event);
     if (h->use_event) cudaEventDestroy(h->use_event);
     tc_destroy(h->tc);
-    for (int i = 0; i < 3; ++i) {
-        cudaFree(h->d_scratch[i]);
-        cudaFree(h->d_z0[i]);
-    }
-    for (int i = 0; i < 5; ++i) cudaFree(h->d_dn[i]);
     if (h->dn_exec) cudaGraphExecDestroy(h->dn_exec);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
     if (h->dn_stream2) cudaStreamDestroy(h->dn_stream2);
     for (int i = 0; i < 2; ++i)
         if (h->dn_ev[i]) cudaEventDestroy(h->dn_ev[i]);
-    for (int i = 0; i < 3; ++i) cudaFree(h->d_pos[i]);
-    cudaFree(h->d_ws);
-    cudaFree(h->d_encrows);
-    cudaFree(h->d_loss_partial);
-    cudaFree(h->d_loss_counter);
-    cudaFree(h->d_loss_totals);
-    for (int i = 0; i < 2; ++i) {
+    for (int i = 0; i < 2; ++i)
         if (h->hs[i]) cudaStreamDestroy(h->hs[i]);
-        if (i == 0 && h->hs_ev) cudaEventDestroy(h->hs_ev);
-        cudaFree(h->d_chunk[i]);
-        cudaFree(h->d_chunk_dist[i]);
-    }
-    delete h;
+    if (h->hs_ev) cudaEventDestroy(h->hs_ev);
+    delete h;      // frees the device buffers
     return 0;
 }
 
@@ -520,8 +472,8 @@ int pndf_set_weights(pndf_handle* h, const float* flat, size_t n) {
     if (!h || !flat) return fail("null argument");
     if (n != param_count(&h->cfg)) return fail("pndf_set_weights: wrong parameter count");
     CUDA_OK(cudaSetDevice(h->cfg.device));
-    CUDA_OK(cudaMemcpy(h->d_flat, flat, n * sizeof(float), cudaMemcpyHostToDevice));
-    if (pack_on_device(h, h->d_flat, nullptr)) return 1;
+    CUDA_OK(cudaMemcpy(h->d_flat.get(), flat, n * sizeof(float), cudaMemcpyHostToDevice));
+    if (pack_on_device(h, h->d_flat.get(), nullptr)) return 1;
     CUDA_OK(cudaStreamSynchronize(nullptr));
     return 0;
 }
@@ -684,34 +636,34 @@ int pndf_project_host(pndf_handle* h, const float* pose_in_host, float* pose_out
         const int64_t chunk = (int64_t)h->num_sms * 4 * kTileM;
         for (int64_t off = 0; off < B; off += chunk) sizes.push_back(std::min(chunk, B - off));
     }
-    const int64_t need = *std::max_element(sizes.begin(), sizes.end());
-    if (h->chunk_poses < need) {
+    const size_t need = (size_t)*std::max_element(sizes.begin(), sizes.end());
+    bool grow = false;
+    for (int i = 0; i < 2; ++i) grow |= h->d_chunk[i].size() < need * 84 || h->d_chunk_dist[i].size() < need;
+    if (grow) {
         CUDA_OK(cudaStreamSynchronize(h->hs[0]));
         CUDA_OK(cudaStreamSynchronize(h->hs[1]));
-        for (int i = 0; i < 2; ++i) {
-            cudaFree(h->d_chunk[i]); cudaFree(h->d_chunk_dist[i]);
-            h->d_chunk[i] = nullptr; h->d_chunk_dist[i] = nullptr;
-            CUDA_OK(cudaMalloc(&h->d_chunk[i], need * 84 * sizeof(float)));
-            CUDA_OK(cudaMalloc(&h->d_chunk_dist[i], need * sizeof(float)));
-        }
-        h->chunk_poses = need;
+        for (int i = 0; i < 2; ++i)
+            if (h->d_chunk[i].reserve(need * 84, "host pipeline chunk") || h->d_chunk_dist[i].reserve(need, "host pipeline chunk distances"))
+                return 1;
     }
     int which = 0;
     int64_t off = 0;
     for (size_t ci = 0; ci < sizes.size(); off += sizes[ci], ++ci, which ^= 1) {
         const int64_t nb = sizes[ci];
         cudaStream_t st = h->hs[which];
-        CUDA_OK(cudaMemcpyAsync(h->d_chunk[which], pose_in_host + off * 84, nb * 84 * sizeof(float), cudaMemcpyHostToDevice, st));
+        float* chunk = h->d_chunk[which].get();
+        float* chunk_dist = h->d_chunk_dist[which].get();
+        CUDA_OK(cudaMemcpyAsync(chunk, pose_in_host + off * 84, nb * 84 * sizeof(float), cudaMemcpyHostToDevice, st));
         KParams p{};
-        p.pose_in = h->d_chunk[which]; p.pose_out = h->d_chunk[which]; p.dist = h->d_chunk_dist[which]; p.B = nb;
+        p.pose_in = chunk; p.pose_out = chunk; p.dist = chunk_dist; p.B = nb;
         p.steps = steps; p.do_step = 1; p.renorm = renorm; p.normalise = 1; p.input_kind = IN_QUAT;
         // the tensor-core path keeps its activations in ONE set of buffers per handle: its launches of consecutive chunks must not
         // overlap (the copies of the two streams still do)
         if (tile == 128 && off > 0) CUDA_OK(cudaStreamWaitEvent(st, h->hs_ev, 0));
         if (launch(h, p, 1, tile, st, 1 + which)) return 1;
         if (tile == 128) CUDA_OK(cudaEventRecord(h->hs_ev, st));
-        CUDA_OK(cudaMemcpyAsync(pose_out_host + off * 84, h->d_chunk[which], nb * 84 * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (dist_host) CUDA_OK(cudaMemcpyAsync(dist_host + off, h->d_chunk_dist[which], nb * sizeof(float), cudaMemcpyDeviceToHost, st));
+        CUDA_OK(cudaMemcpyAsync(pose_out_host + off * 84, chunk, nb * 84 * sizeof(float), cudaMemcpyDeviceToHost, st));
+        if (dist_host) CUDA_OK(cudaMemcpyAsync(dist_host + off, chunk_dist, nb * sizeof(float), cudaMemcpyDeviceToHost, st));
     }
     CUDA_OK(cudaStreamSynchronize(h->hs[0]));
     CUDA_OK(cudaStreamSynchronize(h->hs[1]));
@@ -729,15 +681,8 @@ int pndf_denoise_prior(pndf_handle* h, float* aa_dev, int64_t S, int64_t T, int 
     CUDA_OK(cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t B = S * T;
-    if (h->dn_poses < B) {
-        for (int i = 0; i < 5; ++i) {
-            cudaFree(h->d_dn[i]);
-            h->d_dn[i] = nullptr;
-        }
-        for (int i = 0; i < 3; ++i) CUDA_OK(cudaMalloc(&h->d_dn[i], (size_t)B * 63 * sizeof(float)));
-        for (int i = 3; i < 5; ++i) CUDA_OK(cudaMalloc(&h->d_dn[i], (size_t)B * sizeof(float)));
-        h->dn_poses = B;
-    }
+    for (int i = 0; i < 5; ++i)
+        if (h->d_dn[i].reserve((size_t)B * (i < 3 ? 63 : 1), "denoise loop state")) return 1;
     if (!h->dn_stream2) {
         if (cudaStreamCreateWithFlags(&h->dn_stream2, cudaStreamNonBlocking) != cudaSuccess) h->dn_stream2 = nullptr;
         for (int i = 0; i < 2 && h->dn_stream2; ++i)
@@ -748,12 +693,12 @@ int pndf_denoise_prior(pndf_handle* h, float* aa_dev, int64_t S, int64_t T, int 
         cudaGetLastError();
     }
     if (h->dn_stream2 && ensure_slot(h, 1)) return 1;
-    float* graw = h->d_dn[0];
-    float* m = h->d_dn[1];
-    float* v = h->d_dn[2];
+    float* graw = h->d_dn[0].get();
+    float* m = h->d_dn[1].get();
+    float* v = h->d_dn[2].get();
     // distances are double-buffered (the update prologue of step t reads whole sequences of step t-1 while other CTAs already
     // write step t); the buffers alternate so that the LAST step lands in the caller's array
-    float* dbuf[2] = {dist_dev ? dist_dev : h->d_dn[3], h->d_dn[4]};
+    float* dbuf[2] = {dist_dev ? dist_dev : h->d_dn[3].get(), h->d_dn[4].get()};
     const int nsteps = iterations * steps_per_iter;
     const double b1 = 0.9, b2 = 0.999;
     auto adam_of = [&](int t1, int it) {      // parameters of update number t1 (1-based), loss weight of outer iteration `it`
@@ -901,7 +846,7 @@ int pndf_encoder_tangent(pndf_handle* h, const float* pose_dev, const float* v_d
     if (!h->have_weights) return fail("pndf_set_weights has not been called");
     CUDA_OK(cudaSetDevice(h->cfg.device));
     EncTrainParams p{};
-    p.x = pose_dev; p.v = v_dev; p.encw = h->d_small + h->off_enc; p.zdot_tiles = zdot_tiles_dev; p.B = B;
+    p.x = pose_dev; p.v = v_dev; p.encw = h->d_small.get() + h->off_enc; p.zdot_tiles = zdot_tiles_dev; p.B = B;
     p.normalise = normalise; p.act = h->cfg.enc_act; p.beta = h->cfg.enc_beta; p.use_enc = h->cfg.use_enc;
     if (order_after_weights(h, (cudaStream_t)stream)) return 1;
     enc_tangent_kernel<<<(unsigned)((B + 127) / 128), 128, 0, (cudaStream_t)stream>>>(p);
@@ -921,17 +866,17 @@ int pndf_encoder_param_grads(pndf_handle* h, const float* pose_dev, const float*
     cudaStream_t st = (cudaStream_t)stream;
     CUDA_OK(cudaMemsetAsync(grads_dev, 0, 2 * kEncFloats * sizeof(float), st));
     if (B == 0) return 0;
-    if (ensure_encrows(h, B)) return 1;
     const long long nwarps = ((B + 127) / 128) * 4;
+    if (ensure_encrows(h, nwarps)) return 1;
     EncTrainParams p{};
-    p.x = pose_dev; p.v = v_dev; p.encw = h->d_small + h->off_enc; p.up1 = up_first_dev; p.upt = up_tangent_dev;
-    p.upz = up_second_dev; p.grads = h->d_encrows; p.B = B; p.normalise = normalise; p.act = h->cfg.enc_act;
+    p.x = pose_dev; p.v = v_dev; p.encw = h->d_small.get() + h->off_enc; p.up1 = up_first_dev; p.upt = up_tangent_dev;
+    p.upz = up_second_dev; p.grads = h->d_encrows.get(); p.B = B; p.normalise = normalise; p.act = h->cfg.enc_act;
     p.beta = h->cfg.enc_beta; p.use_enc = 1;
     if (order_after_weights(h, st)) return 1;
     enc_grad_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(p);
     CUDA_OK(cudaGetLastError());
     const int nsets = (up_tangent_dev || up_second_dev) ? 2 : 1;
-    enc_rows_reduce_kernel<<<(nsets * kEncFloats + 255) / 256, 256, 0, st>>>(h->d_encrows, nwarps, nsets, grads_dev);
+    enc_rows_reduce_kernel<<<(nsets * kEncFloats + 255) / 256, 256, 0, st>>>(h->d_encrows.get(), nwarps, nsets, grads_dev);
     CUDA_OK(cudaGetLastError());
     h->launches += 2;
     return 0;
@@ -963,21 +908,14 @@ int pndf_train_losses(pndf_handle* h, const float* dist_dev, const float* dist_g
     if (mode == 0 && grad_dev && !v_dev) return fail("pndf_train_losses: Eikonal term needs the tangent output");
     CUDA_OK(cudaSetDevice(h->cfg.device));
     const int blocks = (int)((B + 255) / 256);
-    if (h->loss_blocks < blocks) {
-        cudaFree(h->d_loss_partial);
-        h->d_loss_partial = nullptr;
-        CUDA_OK(cudaMalloc(&h->d_loss_partial, (size_t)blocks * 2 * sizeof(float)));
-        h->loss_blocks = blocks;
-    }
-    if (!h->d_loss_counter) {
-        CUDA_OK(cudaMalloc(&h->d_loss_counter, sizeof(unsigned int)));
-        CUDA_OK(cudaMemset(h->d_loss_counter, 0, sizeof(unsigned int)));
-        CUDA_OK(cudaMalloc(&h->d_loss_totals, 3 * sizeof(double)));
-        CUDA_OK(cudaMemset(h->d_loss_totals, 0, 3 * sizeof(double)));
-    }
+    // the counter and the totals are zeroed once, when they are allocated: from then on the kernel resets the counter itself, and
+    // the totals on a call with `reset`
+    if (h->d_loss_partial.reserve((size_t)blocks * 2, "loss partial sums") || h->d_loss_counter.reserve(1, "loss counter", true) ||
+        h->d_loss_totals.reserve(3, "loss totals", true))
+        return 1;
     LossParams p{};
     p.dist = dist_dev; p.dist_gt = dist_gt_dev; p.grad = grad_dev; p.coef = coef_dev; p.v = v_dev;
-    p.partial = h->d_loss_partial; p.counter = h->d_loss_counter; p.totals = h->d_loss_totals; p.losses = losses_dev;
+    p.partial = h->d_loss_partial.get(); p.counter = h->d_loss_counter.get(); p.totals = h->d_loss_totals.get(); p.losses = losses_dev;
     p.B = B; p.inv_n = 1.0 / (double)B_total; p.mode = mode; p.l2 = l2; p.reset = reset;
     if (reset && mode == 0) CUDA_OK(cudaMemsetAsync(losses_dev, 0, 3 * sizeof(float), (cudaStream_t)stream));
     train_loss_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(p);
@@ -996,7 +934,8 @@ int pndf_wgrad_accumulate(pndf_handle* h, const float* pose_dev, const float* v_
     if (!h->have_weights) return fail("pndf_set_weights has not been called");
     CUDA_OK(cudaSetDevice(h->cfg.device));
     cudaStream_t st = (cudaStream_t)stream;
-    const size_t n_params = param_count(&h->cfg);
+    const ParamLayout L(h->cfg);
+    const size_t n_params = (size_t)L.total;
     const size_t ws_stride = (n_params + 3) & ~(size_t)3;      // 16-byte aligned workspace slots (vector stores)
     // K-split length: 84 output tiles per split, 2 CTAs per SM -- pick the multiple of 32 poses in [768, 1536] that wastes the
     // least of the last wave (B = 32 768: 864 poses -> 38 splits, 3 192 CTAs = 10.8 waves of 296)
@@ -1013,41 +952,29 @@ int pndf_wgrad_accumulate(pndf_handle* h, const float* pose_dev, const float* v_
         }
     }
     const int ksplits = (int)((B + kc - 1) / kc);
-    if (h->ws_slots < ksplits) {
-        cudaFree(h->d_ws);
-        h->d_ws = nullptr;
-        CUDA_OK(cudaMalloc(&h->d_ws, (size_t)ksplits * ws_stride * sizeof(float)));
-        h->ws_slots = ksplits;
-    }
-    if (h->cfg.use_enc && ensure_encrows(h, B)) return 1;
+    const long long nwarps = ((B + 127) / 128) * 4;      // of the encoder-gradient kernel
+    if (h->d_ws.reserve((size_t)ksplits * ws_stride, "split-K workspace")) return 1;
+    if (h->cfg.use_enc && ensure_encrows(h, nwarps)) return 1;
     static bool attr_set[64] = {};
     if (h->cfg.device < 64 && !attr_set[h->cfg.device]) {
         CUDA_OK(cudaFuncSetAttribute(wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmem));
         attr_set[h->cfg.device] = true;
-    }
-    // flat parameter offsets (reference order): [encoder] W0 b0 W1 b1 ... W6 b6
-    const int in0 = h->cfg.in_dim;
-    const int widths[8] = {in0, 256, 512, 1024, 512, 256, 64, 1};
-    long long off = h->cfg.use_enc ? kEncFloats : 0, w_off[7], b_off[7];
-    for (int l = 0; l < 7; ++l) {
-        w_off[l] = off; off += (long long)widths[l + 1] * widths[l];
-        b_off[l] = off; off += widths[l + 1];
     }
     // export column map (DESIGN.md): layer inputs z_l, adjoints of pre_l
     const int z_col[7] = {0, 128, 384, 896, 1920, 2432, 2688};
     const int a_col[6] = {5120, 4608, 3584, 3072, 2816, 2752};
     WgParams p{};
     p.dump = dump_dev; p.dump_t = dump_t_dev; p.coef = coef_dev; p.up = up_dev; p.w_eik = w_eik_dev; p.uniform = uniform;
-    p.ws = h->d_ws; p.B = B; p.ws_stride = (long long)ws_stride; p.kc = kc; p.slot0 = 0; p.nprob = 6;
+    p.ws = h->d_ws.get(); p.B = B; p.ws_stride = (long long)ws_stride; p.kc = kc; p.slot0 = 0; p.nprob = 6;
     int tiles = 0;
     // big layers first: their CTAs start first inside every K-split
     const int order[6] = {2, 3, 1, 4, 0, 5};
     for (int i = 0; i < 6; ++i) {
         const int l = order[i];
         WgProblem& q = p.prob[i];
-        q.a_col = a_col[l]; q.z_col = z_col[l]; q.n_out = widths[l + 1]; q.n_in = widths[l];
+        q.a_col = a_col[l]; q.z_col = z_col[l]; q.n_out = L.width[l + 1]; q.n_in = L.width[l];
         q.m_tiles = (q.n_out + kWgTile - 1) / kWgTile; q.n_tiles = (q.n_in + kWgTile - 1) / kWgTile;
-        q.tile0 = tiles; q.w_off = w_off[l]; q.b_off = b_off[l];
+        q.tile0 = tiles; q.w_off = L.w_off[l]; q.b_off = L.b_off[l];
         tiles += q.m_tiles * q.n_tiles;
     }
     if (order_after_weights(h, st)) return 1;
@@ -1055,7 +982,7 @@ int pndf_wgrad_accumulate(pndf_handle* h, const float* pose_dev, const float* v_
     CUDA_OK(cudaGetLastError());
     WgLastParams lp{};
     lp.dump = dump_dev; lp.dump_t = dump_t_dev; lp.coef = coef_dev; lp.up = up_dev; lp.w_eik = w_eik_dev; lp.dist = dist_dev;
-    lp.uniform = uniform; lp.ws = h->d_ws; lp.B = B; lp.ws_stride = (long long)ws_stride; lp.w6_off = w_off[6]; lp.b6_off = b_off[6];
+    lp.uniform = uniform; lp.ws = h->d_ws.get(); lp.B = B; lp.ws_stride = (long long)ws_stride; lp.w6_off = L.w_off[6]; lp.b6_off = L.b_off[6];
     lp.kc = kc; lp.slot0 = 0; lp.z6_col = z_col[6]; lp.softplus = (h->cfg.df_act == PNDF_ACT_SOFTPLUS); lp.beta = h->cfg.df_beta;
     wgrad_last_kernel<<<(unsigned)ksplits, 256, 0, st>>>(lp);
     CUDA_OK(cudaGetLastError());
@@ -1063,23 +990,21 @@ int pndf_wgrad_accumulate(pndf_handle* h, const float* pose_dev, const float* v_
     float* enc_part = nullptr;
     if (h->cfg.use_enc) {
         EncTrainParams ep{};
-        ep.x = pose_dev; ep.v = (w_eik_dev || upz_dev) ? v_dev : nullptr; ep.encw = h->d_small + h->off_enc; ep.upz = upz_dev;
+        ep.x = pose_dev; ep.v = (w_eik_dev || upz_dev) ? v_dev : nullptr; ep.encw = h->d_small.get() + h->off_enc; ep.upz = upz_dev;
         ep.g0 = dump_dev + 5376; ep.g0_ld = kDumpRows; ep.coef = coef_dev; ep.uniform = uniform; ep.up = up_dev;
         ep.weik = dump_t_dev ? w_eik_dev : nullptr;
-        ep.grads = h->d_encrows; ep.B = B; ep.normalise = normalise; ep.act = h->cfg.enc_act; ep.beta = h->cfg.enc_beta; ep.use_enc = 1;
+        ep.grads = h->d_encrows.get(); ep.B = B; ep.normalise = normalise; ep.act = h->cfg.enc_act; ep.beta = h->cfg.enc_beta; ep.use_enc = 1;
         enc_grad_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>(ep);
         CUDA_OK(cudaGetLastError());
         const int nsets = (ep.weik || ep.upz) ? 2 : 1;
-        const long long nwarps = ((B + 127) / 128) * 4;
-        enc_part = h->d_encrows + (size_t)2 * h->encrow_warps * kEncFloats;
-        enc_rows_partial_kernel<<<dim3((unsigned)((nsets * kEncFloats + 255) / 256), kEncChunks), 256, 0, st>>>(h->d_encrows, nwarps, nsets, enc_part);
+        enc_part = h->d_encrows.get() + (size_t)2 * nwarps * kEncFloats;      // after this call's per-warp rows (ensure_encrows)
+        enc_rows_partial_kernel<<<dim3((unsigned)((nsets * kEncFloats + 255) / 256), kEncChunks), 256, 0, st>>>(h->d_encrows.get(), nwarps, nsets, enc_part);
         CUDA_OK(cudaGetLastError());
         n_enc_rows = kEncChunks * nsets;     // [set][chunk] rows, summed in this order by the reduce kernel
         h->launches++;
     }
-    wgrad_reduce_kernel<<<(unsigned)((n_params + 255) / 256), 256, 0, st>>>(h->d_ws, ksplits, (long long)ws_stride, (long long)n_params,
-                                                                           h->cfg.use_enc ? kEncFloats : 0, enc_part, n_enc_rows,
-                                                                           grad_flat_dev, overwrite);
+    wgrad_reduce_kernel<<<(unsigned)((n_params + 255) / 256), 256, 0, st>>>(h->d_ws.get(), ksplits, (long long)ws_stride, (long long)n_params,
+                                                                           L.enc_floats, enc_part, n_enc_rows, grad_flat_dev, overwrite);
     CUDA_OK(cudaGetLastError());
     h->launches += 3;
     return 0;
@@ -1100,7 +1025,8 @@ int pndf_adam_step(pndf_handle* h, float* param_flat_dev, const float* grad_flat
     p.bias2_sqrt = (float)std::sqrt(1.0 - std::pow(beta2, (double)step));
     p.one_minus_beta1 = (float)(1.0 - beta1); p.beta2 = (float)beta2; p.one_minus_beta2 = (float)(1.0 - beta2);
     p.eps = (float)eps; p.weight_decay = (float)weight_decay; p.grad_scale = (float)grad_scale;
-    p.pos_a = h->d_pos[0]; p.pos_b = h->d_pos[1]; p.pos_s = h->d_pos[2]; p.wstream = h->d_wstream; p.small = h->d_small;
+    p.pos_a = h->d_pos[0].get(); p.pos_b = h->d_pos[1].get(); p.pos_s = h->d_pos[2].get();
+    p.wstream = h->d_wstream.get(); p.small = h->d_small.get();
     if (write_weights(h, param_flat_dev, st, [&] { adam_step_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(p); })) return 1;
     h->launches++;
     return 0;

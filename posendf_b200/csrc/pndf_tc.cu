@@ -29,6 +29,7 @@
 #include <map>
 #include <vector>
 
+#include "pndf_host.h"
 #include "pndf_kernel.cuh"
 #include "pndf_tc_gemm.cuh"
 
@@ -469,16 +470,18 @@ __global__ void __launch_bounds__(128) tc_head_kernel(const HeadParams p) {
 
 // ------------------------------------------------------------------------------------------------ host side
 struct TcState {
+    explicit TcState(const pndf_config& c) : cfg(c), L(c) {}
     pndf_config cfg;
-    int widths[8];                 // in_dim, 256, 512, 1024, 512, 256, 64, 1
+    ParamLayout L;                 // where W_l sits in the flat parameter vector; L.width = in_dim, 256, 512, 1024, 512, 256, 64, 1
     int kpad[6], ninpad[6];        // K of the forward op l (n_in padded to 32), N of the reverse op l (n_in padded to 128)
-    float *w_hi = nullptr, *w_lo = nullptr;
+    int zw[7];                     // width of the stored activation z_l: z_0 padded to kpad[0], then the layer widths
+    DevBuf<float> w_hi, w_lo;
     long long f_off[6], r_off[6], w_total = 0;
-    long long w_off_flat[6];
-    // activations for `cap` poses (multiple of 128): forward z_0..z_6 (hi, lo), reverse t_5..t_0 (hi, lo), g0, dist
-    long long cap = 0;
-    float* act = nullptr;
-    long long z_off[7], t_off[6], g0_off = 0, dist_off = 0, mask_off[7] = {0, 0, 0, 0, 0, 0, 0}, feat_off = 0, act_floats = 0;
+    // activations, for as many poses (a multiple of 128) as `act` holds act_per_pose floats: forward z_0..z_6 (hi, lo), reverse
+    // t_5..t_0 (hi, lo), g0, dist, encoder features, sign masks.  The offsets are per pose: buffer x of a P-pose allocation starts at
+    // float P * x_off
+    DevBuf<float> act;
+    long long z_off[7], t_off[6], g0_off = 0, dist_off = 0, mask_off[7] = {0, 0, 0, 0, 0, 0, 0}, feat_off = 0, act_per_pose = 0;
     int num_sms = 148;
     // tensor maps of the GEMM launches, keyed by (operand / output addresses, shape): a step repeats the same twelve launches, and
     // six cuTensorMapEncodeTiled calls per launch are host time the 15-launch step of a small batch does not have
@@ -496,74 +499,54 @@ static int tc_check(TcState* s, const char* what) {
 const char* tc_last_error(TcState* s) { return s ? s->err.c_str() : "null tc state"; }
 
 int tc_create(TcState** out, const pndf_config* cfg) {
-    TcState* s = new TcState();
-    s->cfg = *cfg;
-    const int w[8] = {cfg->in_dim, 256, 512, 1024, 512, 256, 64, 1};
-    long long off = cfg->use_enc ? kEncFloats : 0, tot = 0;
-    for (int l = 0; l < 8; ++l) s->widths[l] = w[l];
+    TcState* s = new TcState(*cfg);
+    const int* w = s->L.width;
+    long long tot = 0;
     for (int l = 0; l < 6; ++l) {
         s->kpad[l] = (w[l] + 31) / 32 * 32;
         s->ninpad[l] = (w[l] + 127) / 128 * 128;
-        s->w_off_flat[l] = off;
-        off += (long long)w[l + 1] * w[l] + w[l + 1];
     }
     for (int l = 0; l < 6; ++l) { s->f_off[l] = tot; tot += (long long)w[l + 1] * s->kpad[l]; }
     for (int l = 0; l < 6; ++l) { s->r_off[l] = tot; tot += (long long)s->ninpad[l] * w[l + 1]; }
     s->w_total = tot;
+    s->zw[0] = s->kpad[0];
+    for (int l = 1; l < 7; ++l) s->zw[l] = w[l];
+    long long off = 0;
+    for (int l = 0; l < 7; ++l) { s->z_off[l] = off; off += 2 * s->zw[l]; }
+    for (int l = 0; l < 6; ++l) { s->t_off[l] = off; off += 2 * w[l + 1]; }      // t_l has the width of layer l's output
+    s->g0_off = off; off += 128;
+    s->dist_off = off; off += 1;
+    s->feat_off = off; off += 128;                                                 // fp32 encoder features (forward -> reverse kernel)
+    for (int l = 1; l <= 5; ++l) { s->mask_off[l] = off; off += s->zw[l] / 32; }  // sign bits of the pre-activations of z_1 .. z_5
+    s->act_per_pose = off;
     cudaDeviceGetAttribute(&s->num_sms, cudaDevAttrMultiProcessorCount, cfg->device);
-    if (cudaMalloc(&s->w_hi, tot * sizeof(float)) != cudaSuccess || cudaMalloc(&s->w_lo, tot * sizeof(float)) != cudaSuccess) {
-        tc_destroy(s);
-        return 1;
-    }
-    if (!pndf_tc::encode_fn()) {
-        tc_destroy(s);
+    if (s->w_hi.reserve(tot, "tf32 weights (hi)") || s->w_lo.reserve(tot, "tf32 weights (lo)") || !pndf_tc::encode_fn()) {
+        delete s;
         return 1;
     }
     *out = s;
     return 0;
 }
 
-void tc_destroy(TcState* s) {
-    if (!s) return;
-    cudaFree(s->w_hi);
-    cudaFree(s->w_lo);
-    cudaFree(s->act);
-    delete s;
-}
+void tc_destroy(TcState* s) { delete s; }
 
 int tc_set_weights(TcState* s, const float* flat_dev, cudaStream_t st) {
     SplitParams p{};
-    p.flat = flat_dev; p.hi = s->w_hi; p.lo = s->w_lo; p.total = s->w_total;
+    p.flat = flat_dev; p.hi = s->w_hi.get(); p.lo = s->w_lo.get(); p.total = s->w_total;
     for (int l = 0; l < 6; ++l) {
-        p.w_off[l] = s->w_off_flat[l]; p.f_off[l] = s->f_off[l]; p.r_off[l] = s->r_off[l];
-        p.n_in[l] = s->widths[l]; p.n_out[l] = s->widths[l + 1]; p.k_pad[l] = s->kpad[l]; p.n_in_pad[l] = s->ninpad[l];
-        p.f_tile[l] = (s->widths[l + 1] % 128 == 0) ? 128 : 64;
+        p.w_off[l] = s->L.w_off[l]; p.f_off[l] = s->f_off[l]; p.r_off[l] = s->r_off[l];
+        p.n_in[l] = s->L.width[l]; p.n_out[l] = s->L.width[l + 1]; p.k_pad[l] = s->kpad[l]; p.n_in_pad[l] = s->ninpad[l];
+        p.f_tile[l] = (s->L.width[l + 1] % 128 == 0) ? 128 : 64;
     }
     tc_split_weights_kernel<<<148 * 8, 256, 0, st>>>(p);
     return tc_check(s, "tc_split_weights_kernel launch");
 }
 
-static int ensure_act(TcState* s, long long B);
-int tc_reserve(TcState* s, long long B) { return ensure_act(s, B); }
-static int ensure_act(TcState* s, long long B) {
-    const long long P = (B + 127) / 128 * 128;
-    if (P <= s->cap) return 0;
-    cudaFree(s->act);
-    s->act = nullptr;
-    s->maps.clear();
-    long long off = 0;
-    const int zw[7] = {s->kpad[0], 256, 512, 1024, 512, 256, 64};
-    for (int l = 0; l < 7; ++l) { s->z_off[l] = off; off += 2 * P * zw[l]; }
-    const int tw[6] = {256, 512, 1024, 512, 256, 64};      // t_l has the width of layer l's output
-    for (int l = 0; l < 6; ++l) { s->t_off[l] = off; off += 2 * P * tw[l]; }
-    s->g0_off = off; off += P * 128;
-    s->dist_off = off; off += P;
-    s->feat_off = off; off += P * 128;                                                  // fp32 encoder features (forward -> reverse kernel)
-    for (int l = 1; l <= 5; ++l) { s->mask_off[l] = off; off += P * zw[l] / 32; }      // sign bits of the pre-activations of z_1 .. z_5
-    if (cudaMalloc(&s->act, off * sizeof(float)) != cudaSuccess) return tc_fail(s, "tensor-core path: cannot allocate the activation buffers");
-    if (cudaMemset(s->act, 0, off * sizeof(float)) != cudaSuccess) return tc_fail(s, "cudaMemset failed");
-    s->cap = P;
-    s->act_floats = off;
+int tc_reserve(TcState* s, long long B) {
+    const size_t need = (size_t)((B + 127) / 128 * 128 * s->act_per_pose);
+    if (need <= s->act.size()) return 0;
+    s->maps.clear();      // the cached tensor maps point into the buffer being replaced
+    if (s->act.reserve(need, "tensor-core activations", true)) return tc_fail(s, pndf_last_error());
     return 0;
 }
 
@@ -601,20 +584,23 @@ static int launch_gemm(TcState* s, const float* a_hi, const float* a_lo, long lo
 int tc_run(TcState* s, const KParams& a, int want_grad, cudaStream_t st, int64_t* launches) {
     if (a.input_kind != IN_QUAT && (a.steps != 1 || a.do_step || a.pose_out != nullptr))
         return tc_fail(s, "tensor-core path: axis-angle input is the prior mode (one evaluation, no step)");
-    if (ensure_act(s, a.B)) return 1;
+    if (tc_reserve(s, a.B)) return 1;
     const long long P = (a.B + 127) / 128 * 128;
     const pndf_config& cfg = s->cfg;
     const bool dsoft = cfg.df_act == PNDF_ACT_SOFTPLUS, esoft = cfg.enc_act == PNDF_ACT_SOFTPLUS;
     const float dpar = dsoft ? cfg.df_beta : (cfg.df_act == PNDF_ACT_RELU ? 0.0f : 0.01f);
-    const int zw[7] = {s->kpad[0], 256, 512, 1024, 512, 256, 64};
-    auto zhi = [&](int l) { return s->act + s->z_off[l]; };
-    auto zlo = [&](int l) { return s->act + s->z_off[l] + P * zw[l]; };
-    auto thi = [&](int l) { return s->act + s->t_off[l]; };
-    auto tlo = [&](int l) { return s->act + s->t_off[l] + P * s->widths[l + 1]; };
-    auto maskp = [&](int l) { return reinterpret_cast<uint32_t*>(s->act + s->mask_off[l]); };
-    float* g0 = s->act + s->g0_off;
-    float* featp = s->act + s->feat_off;
-    float* dkeep = s->act + s->dist_off;
+    const int* zw = s->zw;
+    const int* widths = s->L.width;
+    const long long cap = (long long)(s->act.size() / s->act_per_pose);      // poses the activation buffers hold (>= P)
+    float* act = s->act.get();
+    auto zhi = [&](int l) { return act + cap * s->z_off[l]; };
+    auto zlo = [&](int l) { return zhi(l) + P * zw[l]; };
+    auto thi = [&](int l) { return act + cap * s->t_off[l]; };
+    auto tlo = [&](int l) { return thi(l) + P * widths[l + 1]; };
+    auto maskp = [&](int l) { return reinterpret_cast<uint32_t*>(act + cap * s->mask_off[l]); };
+    float* g0 = act + cap * s->g0_off;
+    float* featp = act + cap * s->feat_off;
+    float* dkeep = act + cap * s->dist_off;
     cudaFuncSetAttribute(tc_enc_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc_sm_total<false>());
     cudaFuncSetAttribute(tc_enc_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc_sm_total<true>());
     cudaFuncSetAttribute(tc_enc_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc_sm_total<false>());
@@ -634,9 +620,9 @@ int tc_run(TcState* s, const KParams& a, int want_grad, cudaStream_t st, int64_t
         if (tc_check(s, "tc_enc_kernel (forward) launch")) return 1;
         // ---- forward chain
         for (int l = 0; l < 6; ++l) {
-            const float* bh = s->w_hi + s->f_off[l];
-            const float* bl = s->w_lo + s->f_off[l];
-            const int N = s->widths[l + 1];
+            const float* bh = s->w_hi.get() + s->f_off[l];
+            const float* bl = s->w_lo.get() + s->f_off[l];
+            const int N = widths[l + 1];
             auto fwd = [&](auto fe) {
                 return (N % 128 == 0) ? launch_gemm<128>(s, zhi(l), zlo(l), P, s->kpad[l], bh, bl, N, fe, st)
                                       : launch_gemm<64>(s, zhi(l), zlo(l), P, s->kpad[l], bh, bl, N, fe, st);
@@ -657,9 +643,9 @@ int tc_run(TcState* s, const KParams& a, int want_grad, cudaStream_t st, int64_t
         if (!want_grad) break;
         // ---- reverse chain: op l maps t_l (width n_out[l]) through W_l to the input side (width n_in[l])
         for (int l = 5; l >= 0; --l) {
-            const float* bh = s->w_hi + s->r_off[l];
-            const float* bl = s->w_lo + s->r_off[l];
-            const int K = s->widths[l + 1], N = s->ninpad[l];
+            const float* bh = s->w_hi.get() + s->r_off[l];
+            const float* bl = s->w_lo.get() + s->r_off[l];
+            const int K = widths[l + 1], N = s->ninpad[l];
             int rc;
             if (l > 0) {
                 rc = dsoft ? launch_gemm<128>(s, thi(l), tlo(l), P, K, bh, bl, N, BwdEpi<true>{zhi(l), zlo(l), thi(l - 1), tlo(l - 1), zw[l], dpar, nullptr}, st)
